@@ -9,6 +9,7 @@ Contract (see the task statement):  python bench.py --gpus N --steps K --warmup 
   roofline   : the dominant hot-path kernel, timed alone with CUDA events inside this process
   cpu_baseline: the oracle port of the reference's CPU path (same model, small batch) on the host cores
   --impl reference : only the CPU arm (reference algorithm port), same metric / config
+  --dump-outputs DIR: after the timed steps, what the last timed step computed, as DIR/<name>.npy (see dump_outputs)
 """
 from __future__ import annotations
 
@@ -20,11 +21,13 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
 
 PER_GPU_BATCH = 256           # BASELINE config 3: synthetic ImageNet-shape batch = 256 / GPU
 MODEL, IMG = "vil_small", 224
@@ -319,6 +322,27 @@ def config5_sweep(dev, B=8, img=512, reps=10):
     return out
 
 
+# ------------------------------------------------------------------------------------------ output dump
+DUMP_SAMPLE = 1 << 21        # elements kept of the flattened gradients / parameters (8 MB each in float32)
+
+
+def dump_outputs(out_dir, net, loss, logits):
+    """Write what one training step hands back to its caller, so that two builds can be compared output for output:
+    logits.npy (batch x classes), loss.npy, and grads.npy / params.npy - the gradients and the updated parameters of
+    net.parameters(), flattened in order and sampled at DUMP_SAMPLE fixed (seed 0) positions.  All float32, 17 MB for
+    ViL-Small."""
+    params = list(net.parameters())
+    flat_p = torch.cat([p.detach().reshape(-1) for p in params]).float().cpu()
+    flat_g = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1) for p in params]).float().cpu()
+    n = flat_p.numel()
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values if n > DUMP_SAMPLE else None
+    arrays = {"logits": logits.detach().float().cpu(), "loss": loss.detach().float().cpu(),
+              "params": flat_p if idx is None else flat_p[idx], "grads": flat_g if idx is None else flat_g[idx]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy())
+
+
 # ------------------------------------------------------------------------------------------ CPU arm
 def cpu_training_throughput(steps, warmup, batch=4):
     """The reference's CPU path, restated (oracle port, `chunked_attention` with the hand-written backward
@@ -363,7 +387,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 30)), max(0, min(args.warmup, 3))
+    steps, warmup = args.steps, max(0, min(args.warmup, 3))
     ips, ms, cores, batch = cpu_training_throughput(steps, warmup)
     line = {"impl": "reference", "metric": "images/sec ViL-Small 224x224 training", "value": ips, "unit": "images/sec",
             "n_gpus": args.gpus, "steps": steps, "warmup": warmup, "ms_per_step": ms, "higher_is_better": True,
@@ -391,11 +415,14 @@ def main():
     ap.add_argument("--no-microbench", action="store_true")
     ap.add_argument("--micro-only", action="store_true", help="only the attention-kernel microbench (BASELINE config 2)")
     ap.add_argument("--config5", action="store_true", help="BASELINE config 5: ViL-Base-Deep 512x512 backbone-forward window sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the logits, loss and a fixed sample of the "
+                                                          "gradients and updated parameters of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
-    import __graft_entry__ as ge
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -403,8 +430,8 @@ def main():
         raise RuntimeError("bench.py needs CUDA devices; the hot path has no CPU fallback (use --impl reference for the CPU arm)")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
-    if rank == 0:
-        ge.build()
+    from vision_longformer_b200 import _lib, build_vil
+    _lib.load()                 # built by __graft_entry__.build(); raises when it is missing
     if args.config5:
         sweep = config5_sweep(dev)
         base = next(r for r in sweep if r["w"] == 7 and r["nglo"] == 1)
@@ -424,8 +451,6 @@ def main():
         import torch.distributed as dist
         dist.init_process_group("nccl", device_id=dev)
         dist.barrier()
-    from vision_longformer_b200 import _lib, build_vil
-    _lib.load()
     warmup = max(3, args.warmup)
     steps = args.steps
     B = args.batch
@@ -445,11 +470,12 @@ def main():
 
     def step(x, y):
         with torch.autocast("cuda", dtype=torch.bfloat16):
-            loss = torch.nn.functional.cross_entropy(model(x), y)
+            logits = model(x)
+            loss = torch.nn.functional.cross_entropy(logits, y)
         opt.zero_grad(set_to_none=True)
         loss.backward()
         opt.step()
-        return loss
+        return loss, logits
 
     def sync_all():
         if world > 1:
@@ -474,12 +500,15 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            step(x_dev, y_dev)
+            last_step = step(x_dev, y_dev)
         e1.record()
         sync_all()
     launches = _lib.launch_count() - launches0
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net, *last_step)
+    del last_step
 
     # ---- end-to-end timing: every step's images / labels are copied from PINNED HOST memory inside the timed region and
     # the loss is read back every step.  The copy of step i+1 runs on a side stream while step i computes (double-buffered
@@ -508,7 +537,7 @@ def main():
                 prefetch(i + 1)
             cur.wait_event(ready[i & 1])
             xb, yb = stage[i & 1]
-            loss = step(xb, yb)
+            loss, _ = step(xb, yb)
             freed[i & 1].record(cur)
             last = loss.item()                                # D2H read of the step's result
         return last

@@ -1,8 +1,9 @@
-"""Generate golden vectors by IMPORTING THE UNMODIFIED REFERENCE (/root/reference).
+"""Generate golden vectors by IMPORTING THE UNMODIFIED REFERENCE (a checkout of microsoft/vision-longformer).
 
-Run in the authoring container only (the reference does not travel to the GPU
-box):   python oracle/make_golden.py
-Outputs small fixtures under tests/golden/*.pt which ARE committed.
+    python oracle/make_golden.py <vision-longformer checkout>
+
+Outputs small fixtures under tests/golden/*.pt which ARE committed, so that the
+test-suite never needs the reference itself.
 
 What is pinned
 --------------
@@ -18,6 +19,11 @@ What is pinned
   pinning the stock-PyTorch harness in vision_longformer_b200/msvit.py.
 * `mask_*.pt`  : raw outputs of the three reference mask builders
   (slidingchunk_2d.py:249-318) for the oracle's closed forms.
+* `dropin_reference.pt` : what the reference MsViT and `Long2DSCSelfAttention`
+  expose to a drop-in class (state_dict keys / shapes, public attributes, MAC
+  counts), for tests/test_dropin_reference.py.
+* `reference_fresh_seed.pt` : one more `Long2DSCSelfAttention` forward at a
+  configuration none of the `attn_*.pt` cases uses, for the oracle.
 """
 import os
 import random
@@ -26,7 +32,6 @@ import types
 
 import torch
 
-REF = "/root/reference/src"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
 
 
@@ -57,10 +62,11 @@ def install_timm_shim():
     sys.modules.update({"timm": timm, "timm.models": models, "timm.models.layers": layers})
 
 
-def import_reference():
+def import_reference(checkout):
     install_timm_shim()
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
+    src = os.path.join(os.path.abspath(checkout), "src")
+    if src not in sys.path:
+        sys.path.insert(0, src)
     from models.layers.longformer2d import Long2DSCSelfAttention
     from models.layers import slidingchunk_2d
     from models.msvit import MsViT
@@ -172,15 +178,66 @@ def gen_masks(sc):
     print("wrote masks.pt", len(out))
 
 
-def main():
+# a 224x224 MsViT with two longformer stages (s1) and two dense ones, built the way `build_model` builds ViL
+DROPIN_MSVIT = dict(arch="l1,h1,d48,n1,s1,g1,p4,f7_l2,h3,d96,n1,s1,g1,p2,f7_l3,h3,d192,n2,s0,g1,p2,f7_l4,h6,d384,n1,s0,g0,p2,f7",
+                    img_size=224, num_classes=10, drop_path_rate=0.1, norm_embed=True, sharew=True,
+                    attn_type="longformerhand", sw_exact=0, mode=1, ln_eps=1e-6)
+# public attributes of Long2DSCSelfAttention that the rest of the reference reads
+DROPIN_ATTRS = ("Nglo", "num_heads", "head_dim", "attention_window", "only_glo", "scale", "exact", "rpe")
+
+
+def gen_dropin(Cls, MsViT):
+    """What a drop-in class must reproduce: the stock MsViT's state_dict layout and parameter count, the attributes and
+    the MAC count (compute_macs, longformer2d.py:231-280, at a 56x56 token grid) of each longformer attention, and the
+    state_dict of a non-shared-weight, rpe, exact=1 module."""
+    torch.manual_seed(0)
+    net = MsViT(**DROPIN_MSVIT)
+    attn = []
+    for m in net.modules():
+        if isinstance(m, Cls):
+            m.__flops__ = 0
+            Cls.compute_macs(m, (torch.zeros(1, m.Nglo + 56 * 56, m.num_heads * m.head_dim),), None)
+            attn.append(dict({a: getattr(m, a) for a in DROPIN_ATTRS}, macs_56x56=m.__flops__))
+    sd = net.state_dict()
+    first = {}                  # sharew: the global-token Linears ARE the local ones, so their entries share storage
+    tied = {k: first.setdefault(v.data_ptr(), k) for k, v in sd.items()}
+    msvit = dict(kwargs=DROPIN_MSVIT, attn=attn, n_params=sum(p.numel() for p in net.parameters()),
+                 state_dict={k: (tuple(v.shape), v.dtype) for k, v in sd.items()}, tied={k: t for k, t in tied.items() if t != k})
+    kw = dict(dim=48, num_heads=3, qkv_bias=True, w=4, nglo=2, sharew=False, rpe=True, exact=1, mode=0)
+    torch.manual_seed(1)
+    ref = Cls(autograd=False, **kw)
+    nonshared = dict(kwargs=kw, state_dict={k: v.detach().clone() for k, v in ref.state_dict().items()})
+    torch.save(dict(msvit=msvit, nonshared=nonshared), os.path.join(OUT, "dropin_reference.pt"))
+    print("wrote dropin_reference.pt  attn modules=%d" % len(attn))
+
+
+def gen_fresh_seed(Cls):
+    """Float64 eval forward at a configuration (w=3, two global tokens, rpe, separate global weights, 8x10) that the attn_*
+    cases do not cover."""
+    torch.manual_seed(1234)
+    kw = dict(dim=24, num_heads=2, w=3, nglo=2, exact=0, rpe=True, sharew=False, qkv_bias=True)
+    ref = Cls(autograd=False, **kw).double().eval()
+    x = torch.randn(2, 2 + 8 * 10, 24, dtype=torch.float64)
+    with torch.no_grad():
+        y = ref(x, 8, 10)
+    out = dict(kwargs=kw, nx=8, ny=10, state_dict={k: v.detach().clone() for k, v in ref.state_dict().items()}, x=x, y=y)
+    torch.save(out, os.path.join(OUT, "reference_fresh_seed.pt"))
+    print("wrote reference_fresh_seed.pt  y.norm=%.4f" % y.norm().item())
+
+
+def main(checkout):
     os.makedirs(OUT, exist_ok=True)
-    Cls, sc, MsViT = import_reference()
+    Cls, sc, MsViT = import_reference(checkout)
     gen_masks(sc)
     for name, (B, nx, ny, kw, pick) in ATTN_CASES.items():
         gen_attn(name, B, nx, ny, kw, pick, Cls)
     for name, kw in MSVIT_CASES.items():
         gen_msvit(name, kw, MsViT)
+    gen_dropin(Cls, MsViT)
+    gen_fresh_seed(Cls)
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        sys.exit(__doc__)
+    main(sys.argv[1])

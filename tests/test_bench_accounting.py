@@ -61,3 +61,29 @@ def test_committed_ncu_traffic_is_close_to_the_algorithmic_bytes():
             continue
         algo = 256 * b * factor[name]
         assert 0.75 * algo < rec["dram_bytes"] < 1.30 * algo, (key, rec["dram_bytes"], algo)
+
+
+def test_dump_outputs_writes_the_step_results(tmp_path, monkeypatch):
+    """--dump-outputs: float32 .npy files of the logits, loss and a fixed sample of the gradients / updated parameters."""
+    import numpy as np
+    import torch
+    from oracle.vil_oracle import OracleLong2DSCSelfAttention
+    from vision_longformer_b200 import build_vil
+    torch.manual_seed(0)
+    net = build_vil("l1,h2,d16,n1,s1,g1,p4,f4,a0_l2,h2,d32,n1,s1,g1,p2,f4_l3,h2,d32,n1,s0,g1,p2,f7", img_size=32,
+                    num_classes=7, attn_cls=OracleLong2DSCSelfAttention)
+    logits = net(torch.randn(2, 3, 32, 32))
+    loss = torch.nn.functional.cross_entropy(logits, torch.tensor([1, 5]))
+    loss.backward()
+    n = sum(p.numel() for p in net.parameters())
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", n // 3)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), net, loss, logits)
+    got = {f: np.load(tmp_path / "a" / f"{f}.npy") for f in ("logits", "loss", "grads", "params")}
+    assert all(a.dtype == np.float32 for a in got.values())
+    assert got["logits"].shape == (2, 7) and got["loss"].shape == () and got["grads"].shape == got["params"].shape == (n // 3,)
+    assert np.array_equal(got["logits"], logits.detach().numpy()) and got["loss"] == loss.item()
+    flat = torch.cat([p.detach().reshape(-1) for p in net.parameters()]).numpy()
+    assert np.isin(got["params"], flat).all() and np.abs(got["grads"]).sum() > 0
+    for f, a in got.items():                         # the sample positions are fixed
+        assert np.array_equal(a, np.load(tmp_path / "b" / f"{f}.npy")), f

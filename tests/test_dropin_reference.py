@@ -1,106 +1,83 @@
-"""The reference-side binding of INTEGRATION.md section 1, applied to the IMPORTED, UNMODIFIED reference.
+"""The reference-side binding of INTEGRATION.md section 1, checked against what the UNMODIFIED reference exposes.
 
-CPU part (authoring container only - /root/reference does not travel to the GPU box): build the reference's own
-`MsViT` (src/models/msvit.py:343) with `make_dropin_class(Long2DSCSelfAttention)` bound at the seam the reference
-uses (`AttnBlock.__init__`, msvit.py:269-276), and check everything the reference does with that class without
-running it: construction, `isinstance` (msvit.py:532-541 `reset_vil_mode`), `compute_macs`
-(longformer2d.py:231-280), state_dict round trips with a stock reference model.
+CPU part: `make_dropin_class` bound to a stand-in base class with the reference's constructor signature, placed at the
+attention seam of the MsViT harness (`AttnBlock.__init__`, reference msvit.py:269-276), against the stock reference
+`MsViT` (src/models/msvit.py:343) and `Long2DSCSelfAttention` as recorded by oracle/make_golden.py
+(tests/golden/dropin_reference.pt): construction, state_dict layout and round trips, `reset_vil_mode`
+(msvit.py:532-541), the public attributes and `compute_macs` (longformer2d.py:231-280).
 
-GPU part (no reference on the box): the same class factory against a stand-in base class with the reference's
-constructor signature, run forward + backward and compared with the plain B200 module.
+GPU part: the same class factory run forward + backward and compared with the plain B200 module.
 """
-import os
-
 import pytest
 import torch
 from torch import nn
 
-from vision_longformer_b200 import B200Long2DSCSelfAttention, make_dropin_class
-
-REF_SRC = "/root/reference/src"
-needs_ref = pytest.mark.skipif(not os.path.isdir(REF_SRC), reason="the reference tree only exists in the authoring container")
-
-TINY = "l1,h1,d48,n1,s1,g1,p4,f7_l2,h3,d96,n1,s1,g1,p2,f7_l3,h3,d192,n2,s0,g1,p2,f7_l4,h6,d384,n1,s0,g0,p2,f7"
-
-
-def _reference():
-    from oracle.make_golden import import_reference
-    Long2DSCSelfAttention, _, MsViT = import_reference()
-    import models.msvit as ref_msvit
-    return Long2DSCSelfAttention, MsViT, ref_msvit
-
-
-def _build(MsViT, **kw):
-    torch.manual_seed(0)
-    args = dict(arch=TINY, img_size=224, num_classes=10, drop_path_rate=0.1, norm_embed=True, sharew=True,
-                attn_type="longformerhand", sw_exact=0, mode=1, ln_eps=1e-6)
-    args.update(kw)
-    return MsViT(**args)
-
-
-@needs_ref
-def test_dropin_class_binds_into_reference_msvit(monkeypatch):
-    Long2DSCSelfAttention, MsViT, ref_msvit = _reference()
-    stock = _build(MsViT)
-    DropIn = make_dropin_class(Long2DSCSelfAttention)
-    assert issubclass(DropIn, Long2DSCSelfAttention) and issubclass(DropIn, B200Long2DSCSelfAttention)
-    # INTEGRATION.md section 1: "or replace the 'longformerhand' branch outright" - the branch looks the class up by name
-    monkeypatch.setattr(ref_msvit, "Long2DSCSelfAttention", DropIn)
-    net = _build(MsViT)
-    attn = [m for m in net.modules() if isinstance(m, Long2DSCSelfAttention)]
-    assert len(attn) == 2 and all(type(m) is DropIn for m in attn)                  # the two s1 stages
-    assert all(m.forward.__func__ is B200Long2DSCSelfAttention.forward for m in attn)
-    # one parameter set only (the reference constructor must not have run a second time)
-    assert sorted(net.state_dict().keys()) == sorted(stock.state_dict().keys())
-    assert sum(p.numel() for p in net.parameters()) == sum(p.numel() for p in stock.parameters())
-    # checkpoints flow both ways
-    net.load_state_dict(stock.state_dict(), strict=True)
-    stock.load_state_dict(net.state_dict(), strict=True)
-    for k, v in stock.state_dict().items():
-        assert torch.equal(v, net.state_dict()[k]), k
-    # reset_vil_mode finds the modules through isinstance(…, Long2DSCSelfAttention)  (msvit.py:532-541)
-    net.reset_vil_mode(0)
-    assert all(m.mode == 0 for m in attn)
-    net.reset_vil_mode(-1)
-    assert all(m.mode == -1 for m in attn)
-    # public attributes read elsewhere in the reference
-    ref_attn = [m for m in stock.modules() if isinstance(m, Long2DSCSelfAttention)]
-    for a, b in zip(attn, ref_attn):
-        for name in ("Nglo", "num_heads", "head_dim", "attention_window", "only_glo", "scale", "exact", "rpe"):
-            assert getattr(a, name) == getattr(b, name), name
-        assert a.query is a.query_global and a.kv is a.kv_global and a.proj is a.proj_global      # sharew
-    # the MAC-counting hook gives the reference's number (longformer2d.py:231-280)
-    for a, b in zip(attn, ref_attn):
-        x = torch.zeros(1, a.Nglo + 56 * 56, a.num_heads * a.head_dim)
-        a.__flops__, b.__flops__ = 0, 0
-        type(a).compute_macs(a, (x,), None)
-        type(b).compute_macs(b, (x,), None)
-        assert a.__flops__ == b.__flops__ and a.__flops__ > 0
-    # no CPU path: the reference MsViT with the B200 class refuses CPU tensors loudly
-    with pytest.raises(RuntimeError, match="no CPU"):
-        net.eval()(torch.zeros(1, 3, 224, 224))
-
-
-@needs_ref
-def test_dropin_nonshared_weights_and_rpe_state_dict():
-    Long2DSCSelfAttention, _, _ = _reference()
-    DropIn = make_dropin_class(Long2DSCSelfAttention)
-    kw = dict(dim=48, num_heads=3, qkv_bias=True, w=4, nglo=2, sharew=False, rpe=True, exact=1, mode=0)
-    torch.manual_seed(1)
-    ref = Long2DSCSelfAttention(autograd=False, **kw)
-    mod = DropIn(autograd=False, **kw)
-    assert sorted(mod.state_dict().keys()) == sorted(ref.state_dict().keys())
-    mod.load_state_dict(ref.state_dict(), strict=True)
-    assert torch.equal(mod.relative_position_index, ref.relative_position_index)
-    assert mod.query is not mod.query_global
+from tests.util import load_golden
+from vision_longformer_b200 import B200Long2DSCSelfAttention, MsViT, make_dropin_class
 
 
 class _StandIn(nn.Module):
-    """Same constructor signature as the reference class (longformer2d.py:13-14); used where the reference is absent."""
+    """Same constructor signature as the reference class (longformer2d.py:13-14)."""
 
     def __init__(self, dim, num_heads=8, qkv_bias=False, qk_scale=None, attn_drop=0., proj_drop=0., w=7, d=1,
                  autoregressive=False, sharew=False, nglo=1, only_glo=False, exact=0, autograd=False, rpe=False, mode=0):
         raise AssertionError("the base-class constructor must never run in the drop-in class")
+
+
+def _tied(sd):
+    """{key: the first key sharing its storage} for the state_dict entries that alias an earlier one."""
+    first = {}
+    return {k: t for k, t in ((k, first.setdefault(v.data_ptr(), k)) for k, v in sd.items()) if t != k}
+
+
+def test_dropin_class_binds_into_reference_msvit():
+    gold = load_golden("dropin_reference.pt")["msvit"]
+    DropIn = make_dropin_class(_StandIn)
+    torch.manual_seed(0)
+    net = MsViT(attn_cls=DropIn, **gold["kwargs"])
+    attn = [m for m in net.modules() if isinstance(m, _StandIn)]
+    assert len(attn) == len(gold["attn"]) == 2 and all(type(m) is DropIn for m in attn)      # the two s1 stages
+    assert all(m.forward.__func__ is B200Long2DSCSelfAttention.forward for m in attn)
+    # one parameter set only, laid out like the stock reference model's
+    sd = net.state_dict()
+    assert {k: (tuple(v.shape), v.dtype) for k, v in sd.items()} == gold["state_dict"]
+    assert sum(p.numel() for p in net.parameters()) == gold["n_params"]
+    assert _tied(sd) == gold["tied"]                    # sharew: the global-token Linears are the local ones
+    # checkpoints flow both ways: a checkpoint with the reference's layout loads strictly and reads back unchanged
+    gen = torch.Generator().manual_seed(0)
+    ckpt = {k: torch.randn(shape, generator=gen).to(dtype) for k, (shape, dtype) in gold["state_dict"].items()}
+    ckpt.update({k: ckpt[t] for k, t in gold["tied"].items()})
+    net.load_state_dict(ckpt, strict=True)
+    for k, v in net.state_dict().items():
+        assert torch.equal(v, ckpt[k]), k
+    # reset_vil_mode reaches every longformer attention  (msvit.py:532-541)
+    net.reset_vil_mode(0)
+    assert all(m.mode == 0 for m in attn)
+    net.reset_vil_mode(-1)
+    assert all(m.mode == -1 for m in attn)
+    # public attributes read elsewhere in the reference, and the reference's MAC count (longformer2d.py:231-280)
+    for a, ref in zip(attn, gold["attn"]):
+        for name, want in ref.items():
+            if name != "macs_56x56":
+                assert getattr(a, name) == want, name
+        assert a.query is a.query_global and a.kv is a.kv_global and a.proj is a.proj_global      # sharew
+        a.__flops__ = 0
+        type(a).compute_macs(a, (torch.zeros(1, a.Nglo + 56 * 56, a.num_heads * a.head_dim),), None)
+        assert a.__flops__ == ref["macs_56x56"] > 0
+    # no CPU path: the MsViT with the B200 class refuses CPU tensors loudly
+    with pytest.raises(RuntimeError, match="no CPU"):
+        net.eval()(torch.zeros(1, 3, 224, 224))
+
+
+def test_dropin_nonshared_weights_and_rpe_state_dict():
+    gold = load_golden("dropin_reference.pt")["nonshared"]
+    DropIn = make_dropin_class(_StandIn)
+    torch.manual_seed(1)
+    mod = DropIn(autograd=False, **gold["kwargs"])
+    assert sorted(mod.state_dict().keys()) == sorted(gold["state_dict"].keys())
+    assert torch.equal(mod.relative_position_index, gold["state_dict"]["relative_position_index"])
+    mod.load_state_dict(gold["state_dict"], strict=True)
+    assert mod.query is not mod.query_global
 
 
 def test_dropin_mro_never_runs_the_base_constructor():

@@ -1,14 +1,10 @@
 """CPU: pin the oracle (oracle/vil_oracle.py) against golden vectors produced by
 the UNMODIFIED reference (oracle/make_golden.py) and against itself."""
-import os
-
 import pytest
 import torch
 
 from oracle import vil_oracle as vo
 from tests.util import attn_cases, load_attn, load_golden, load_state, relerr
-
-REF_PRESENT = os.path.isdir("/root/reference/src")
 
 
 def run_module(gold, dense):
@@ -89,15 +85,10 @@ def test_dense_and_chunked_agree(cfg):
         assert relerr(a, b) < 1e-11
 
 
-@pytest.mark.skipif(not REF_PRESENT, reason="reference tree only exists in the authoring container")
-def test_oracle_against_live_reference_fresh_seed():
-    """Beyond the committed vectors: a fresh random configuration against the imported reference."""
-    from oracle.make_golden import import_reference
-    Cls, _, _ = import_reference()
-    torch.manual_seed(1234)
-    kw = dict(dim=24, num_heads=2, w=3, nglo=2, exact=0, rpe=True, sharew=False, qkv_bias=True)
-    ref = Cls(autograd=False, **kw).double().eval()
-    mine = vo.OracleLong2DSCSelfAttention(**kw).double().eval()
-    mine.load_state_dict(ref.state_dict())
-    x = torch.randn(2, 2 + 8 * 10, 24, dtype=torch.float64)
-    assert relerr(mine(x, 8, 10), ref(x, 8, 10)) < 1e-13
+def test_oracle_against_reference_fresh_seed():
+    """Beyond the attn_* cases: a configuration none of them uses (w=3, two global tokens, rpe, separate global
+    weights, 8x10), against the reference's float64 forward."""
+    gold = load_golden("reference_fresh_seed.pt")
+    mine = vo.OracleLong2DSCSelfAttention(**gold["kwargs"]).double().eval()
+    mine.load_state_dict(gold["state_dict"])
+    assert relerr(mine(gold["x"], gold["nx"], gold["ny"]), gold["y"]) < 1e-13

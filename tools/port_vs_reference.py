@@ -1,7 +1,7 @@
 """Cost of the oracle PORT (bench.py's CPU arm) relative to the real, unmodified reference MsViT on identical cores.
-Runs in the authoring container only (imports /root/reference through oracle/make_golden.py's timm shim) and writes
-profiles/r02_port_vs_reference.json, which bench.py attaches to `cpu_baseline`.
-usage: python tools/port_vs_reference.py [threads]"""
+Imports the reference checkout through oracle/make_golden.py's timm shim and writes profiles/r02_port_vs_reference.json,
+which bench.py attaches to `cpu_baseline`.
+usage: python tools/port_vs_reference.py <vision-longformer checkout> [threads]"""
 import json
 import os
 import sys
@@ -15,9 +15,9 @@ from oracle.make_golden import import_reference  # noqa: E402
 from oracle.vil_oracle import OracleLong2DSCSelfAttention  # noqa: E402
 from vision_longformer_b200 import ARCHS, build_vil  # noqa: E402
 
-threads = int(sys.argv[1]) if len(sys.argv) > 1 else min(os.cpu_count() or 1, 16)
+threads = int(sys.argv[2]) if len(sys.argv) > 2 else min(os.cpu_count() or 1, 16)
 torch.set_num_threads(threads)
-_, _, RefMsViT = import_reference()
+_, _, RefMsViT = import_reference(sys.argv[1])
 B, IMG = 4, 224
 
 

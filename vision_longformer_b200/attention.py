@@ -191,8 +191,8 @@ def make_dropin_class(reference_cls):
 
     MRO = (B200DropIn, B200Long2DSCSelfAttention, reference_cls, nn.Module): constructor, `forward`, `compute_macs`
     resolve to the B200 module (whose __init__ calls nn.Module.__init__ directly, so the reference constructor never
-    runs); the reference class only contributes its identity.  Pinned by tests/test_dropin_reference.py against the
-    imported, unmodified reference MsViT."""
+    runs); the reference class only contributes its identity.  Pinned by tests/test_dropin_reference.py against what
+    the unmodified reference MsViT exposes (tests/golden/dropin_reference.pt)."""
     class B200DropIn(B200Long2DSCSelfAttention, reference_cls):
         pass
     B200DropIn.__name__ = B200DropIn.__qualname__ = "B200" + reference_cls.__name__
